@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- rendered frames/sec of the ENeRF render-time hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c4|c5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 Workloads (BASELINE.json configs; one "step" = one full frame through the drop-in Network.forward):
@@ -199,7 +199,9 @@ def run_reference_arm(args, rank):
         return
     cfg, net, batch, wl = build_problem(args.workload)
     sd = {k: v.clone() for k, v in net.state_dict().items()}
-    fps, _, n_thr, frames = cpu_reference_run(wl["kind"], cfg, sd, batch, args.steps, warmup=args.warmup)
+    fps, out, n_thr, frames = cpu_reference_run(wl["kind"], cfg, sd, batch, args.steps, warmup=args.warmup)
+    if args.dump_outputs:
+        dump_outputs(host_outputs(out), args.dump_outputs)
     line = {
         "impl": "reference", "metric": wl["metric"], "value": fps, "unit": "frames/s", "n_gpus": args.gpus, "steps": frames,
         "warmup": min(args.warmup, 2), "ms_per_step": 1000.0 / fps, "higher_is_better": True, "scaling": "weak",
@@ -240,6 +242,39 @@ def to_dev(batch, dev):
     return {k: (v.to(dev) if torch.is_tensor(v) and k != "bbox" else v) for k, v in batch.items()}
 
 
+DUMP_BYTES = 60 * 10**6       # array data of --dump-outputs: keeps the directory under 64 MB with the .npy headers
+
+
+def host_outputs(out):
+    """The tensors of a forward's output dict on the host: float64 stays float64 and integer outputs become float64
+    (exact), everything else float32."""
+    res = {}
+    for k, v in out.items():
+        if torch.is_tensor(v):
+            v = v.detach().cpu()
+            wide = v.dtype == torch.float64 or not (v.is_floating_point() or v.dtype == torch.bool)
+            res[k] = v.double() if wide else v.float()
+    return res
+
+
+def dump_outputs(outs, path):
+    """Writes every array of ``outs`` as <path>/<name>.npy.  When they hold more than DUMP_BYTES together, each array is
+    cut to the same fraction of its elements: flattened, at sorted indices drawn with a fixed seed, so that runs and
+    builds with the same arguments dump the same elements."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    total = sum(v.numel() * v.element_size() for v in outs.values())
+    frac = min(1.0, DUMP_BYTES / total) if total else 1.0
+    for k, v in outs.items():
+        if frac < 1.0:
+            flat = v.reshape(-1)
+            idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:int(flat.numel() * frac)]
+            v = flat[idx.sort().values]
+        np.save(os.path.join(path, k + ".npy"), v.numpy())
+    print(f"[bench] {len(outs)} output(s) written to {path}" + (f" (seeded sample of {frac:.3f} of each)" if frac < 1.0 else ""),
+          file=sys.stderr)
+
+
 def timed_events(fn, steps, flush_buf=None):
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
     for a, b in ev:
@@ -265,7 +300,11 @@ def main():
     ap.add_argument("--inflight", type=int, default=4, help="frames rendered concurrently per GPU (one CUDA graph + stream each); "
                     "1 = strictly one frame at a time (latency mode)")
     ap.add_argument("--host-rays", type=int, default=0, help="1: ship rays_1 from the host like the reference's data layer (default: generate on device)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the output tensors of the last one as DIR/<name>.npy "
+                    "(float32 / float64, 64 MB at most: larger outputs are replaced by a fixed seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     from enerf_b200 import dist as edist
@@ -357,13 +396,20 @@ def main():
         return t.tolist()
 
     # ---- headline: device-resident throughput ----
+    last = {}
+
+    def timed_step():
+        last["out"] = step()
+
     for _ in range(args.warmup):
         step()
     sync_all()
     with ClockSampler(local) as clk:
         sync_all()
-        ev = timed_events(step, args.steps, flush_buf)
+        ev = timed_events(timed_step, args.steps, flush_buf)
         sync_all()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(host_outputs(last["out"]), args.dump_outputs)
     times = [a.elapsed_time(b) for a, b in ev]
     (total_ms,) = max_over_ranks([sum(times)])
     frames_per_step = nfl * world

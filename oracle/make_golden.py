@@ -1,4 +1,4 @@
-"""TEST INFRASTRUCTURE -- mint tests/golden/*.pt by running the UNMODIFIED reference on CPU.
+"""TEST INFRASTRUCTURE -- mint tests/golden/*.pt and tests/golden/boundary_*.json by running the UNMODIFIED reference on CPU.
 
 Usage (authoring container only; needs /root/reference or $ENERF_REF):
     python oracle/make_golden.py            # writes every case listed in CASES
@@ -65,6 +65,50 @@ CASES = {
 }
 
 
+# the plugin seam (tests/test_reference_boundary.py): variant -> (yaml, cfg opts, the reference's own module for that cfg)
+BOUNDARY = {
+    "network": ("configs/enerf/dtu_pretrain.yaml", [], "lib.networks.enerf.network"),
+    "network_human": ("configs/enerf/zjumocap_eval.yaml", [], "lib.networks.enerf.network_human"),
+    "network_composite": ("configs/enerf/enerf_outdoor/actor1.yaml", ["num_fg_layers", "2"], "lib.networks.enerf.network_composite"),
+}
+
+
+def state_dict_digest(sd):
+    """[key, shape, dtype, sha256 of the raw bytes] per entry, in state_dict order."""
+    import hashlib
+    return [[k, list(v.shape), str(v.dtype).replace("torch.", ""), hashlib.sha256(v.contiguous().numpy().tobytes()).hexdigest()]
+            for k, v in sd.items()]
+
+
+def run_boundary_case(variant):
+    """The cfg keys the reference's Network reads after its yaml is merged (``enerf``, and ``num_fg_layers`` where the
+    yaml sets it) and the digest of the reference Network's initial state_dict under torch.manual_seed(0)."""
+    import importlib
+    import json
+    import torch
+    from oracle.ref_loader import load_reference
+
+    yaml, opts, module = BOUNDARY[variant]
+    cfg, _ = load_reference(yaml, opts)
+
+    def plain(node):
+        return {k: plain(v) for k, v in node.items()} if isinstance(node, dict) else (list(node) if isinstance(node, tuple) else node)
+
+    keep = {"enerf": plain(cfg.enerf)}
+    if "num_fg_layers" in cfg:
+        keep["num_fg_layers"] = int(cfg.num_fg_layers)
+    torch.manual_seed(0)
+    net = importlib.import_module(module).Network()
+    fixture = {"variant": variant, "yaml": yaml, "opts": opts, "reference_module": module, "reference_commit": "5a084e9",
+               "torch": torch.__version__, "cfg": keep, "state_dict": state_dict_digest(net.state_dict())}
+    path = os.path.join(_ROOT, "tests", "golden", f"boundary_{variant}.json")
+    entries = fixture.pop("state_dict")
+    with open(path, "w") as f:               # one state_dict entry per line
+        f.write(json.dumps(fixture)[:-1] + ', "state_dict": [\n' + ",\n".join(json.dumps(e) for e in entries) + "\n]}\n")
+    fixture["state_dict"] = entries
+    print(variant, "->", path, os.path.getsize(path) // 1024, "KiB;", len(fixture["state_dict"]), "state_dict entries")
+
+
 def run_composite_case(name):
     """network_composite has no per-stage hooks worth stashing: outputs + a few layer intermediates
     recomputed with the reference's own functions."""
@@ -100,6 +144,8 @@ def run_composite_case(name):
 
 
 def run_case(name):
+    if name.startswith("boundary_"):
+        return run_boundary_case(name[len("boundary_"):])
     if CASES[name].get("composite"):
         return run_composite_case(name)
     import torch
@@ -163,5 +209,5 @@ if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "--one":
         run_case(sys.argv[2])
     else:
-        for n in (sys.argv[1:] or list(CASES)):
+        for n in (sys.argv[1:] or list(CASES) + [f"boundary_{v}" for v in BOUNDARY]):
             subprocess.check_call([sys.executable, os.path.abspath(__file__), "--one", n])

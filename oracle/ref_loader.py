@@ -1,9 +1,7 @@
 """TEST INFRASTRUCTURE -- imports the unmodified reference (zju3dv/ENeRF) on CPU.
 
-Only usable where a reference tree exists ($ENERF_REF or /root/reference); the GPU box has none,
-so nothing in the `-m gpu` tests, smoke() or bench.py calls this.  It is used by
-`oracle/make_golden.py` (to mint tests/golden/*.pt) and by `tests/test_reference_boundary.py` (the reference's own
-`make_network(cfg)` loading the drop-in modules), which skips when the tree is absent.
+Only usable where a reference tree exists (see find_reference), so no test, smoke() or bench.py calls this.
+It is used by `oracle/make_golden.py` to mint tests/golden/*.pt and tests/golden/boundary_*.json.
 
 What it does (SURVEY.md section 8c): puts two shims on sys.path (kornia.utils.create_meshgrid,
 imp.load_source), sets $workspace (lib/config/config.py:10), fakes argv before `import lib.config`

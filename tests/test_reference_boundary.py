@@ -1,12 +1,13 @@
 """The drop-in seam, exercised the way the reference itself does it (SURVEY.md section 8b, VERDICT r1 item 7):
-``lib/networks/make_network.py:5-9`` executes the file named by ``cfg.network_module`` with ``imp.load_source`` and
-calls ``Network()`` with no arguments.  Pointing ``network_module`` at /root/repo/enerf_b200/network{,_human,_composite}
-(a dot-free value resolves to ``<value>.py``, lib/config/config.py:166-168) must yield a module whose state_dict is
-key-for-key / shape-for-shape the reference's own, loads the reference's weights with strict=True, and reads the
-same global ``lib.config.cfg``.
+``lib/networks/make_network.py:5-9`` executes the file named by ``cfg.network_path`` with
+``imp.load_source(cfg.network_module, cfg.network_path)`` and calls ``Network()`` with no arguments.  Pointing it at
+enerf_b200/network{,_human,_composite}.py must yield a module whose state_dict is key-for-key / shape-for-shape the
+reference's own, with the same initial values under the same seed, that loads a state_dict of the reference's layout
+with strict=True, and that reads the same global ``lib.config.cfg``.
 
-Needs the reference tree ($ENERF_REF or /root/reference): skipped on the GPU box.  One subprocess per variant because
-the reference builds its cfg at import time from argv (lib/config/config.py:191-201)."""
+What the reference produced for each variant (its merged cfg keys and the digest of its Network's initial
+state_dict) is stored in tests/golden/boundary_<variant>.json, minted by ``oracle/make_golden.py boundary_<variant>``.
+One subprocess per variant because the plugin reads the process-global ``lib.config.cfg``."""
 import os
 import subprocess
 import sys
@@ -14,37 +15,39 @@ import sys
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
-from oracle.ref_loader import find_reference  # noqa: E402
 
-VARIANTS = {
-    "network": ("configs/enerf/dtu_pretrain.yaml", "lib.networks.enerf.network", []),
-    "network_human": ("configs/enerf/zjumocap_eval.yaml", "lib.networks.enerf.network_human", []),
-    "network_composite": ("configs/enerf/enerf_outdoor/actor1.yaml", "lib.networks.enerf.network_composite", ["num_fg_layers", "2"]),
-}
+VARIANTS = ["network", "network_composite", "network_human"]
 
 CHILD = r'''
-import os, sys, torch
+import json, os, sys, types, torch
 sys.path.insert(0, {root!r})
-from oracle.ref_loader import load_reference
+sys.path.insert(0, os.path.join({root!r}, "oracle", "shims"))
+from enerf_b200.config import Node
+from oracle.make_golden import state_dict_digest
+fx = json.load(open(os.path.join({root!r}, "tests", "golden", "boundary_" + {variant!r} + ".json")))
+
+def node(v):
+    return Node({{k: node(x) for k, x in v.items()}}) if isinstance(v, dict) else v
+
 ours = os.path.join({root!r}, "enerf_b200", {variant!r})
-cfg, mods = load_reference({yaml!r}, ["network_module", ours] + {opts!r})
-assert cfg.network_module == ours and cfg.network_path == ours + ".py", (cfg.network_module, cfg.network_path)
-import importlib
-from lib.networks import make_network                      # the reference's own factory (lib/networks/make_network.py)
+cfg = node(fx["cfg"])
+cfg.network_module, cfg.network_path = ours, ours + ".py"
+lib_config = types.ModuleType("lib.config")                # the reference's global cfg, as its run.py leaves it
+lib_config.cfg = cfg
+sys.modules["lib.config"] = lib_config
+import imp
 torch.manual_seed(0)
-net = make_network(cfg)
+net = imp.load_source(cfg.network_module, cfg.network_path).Network()   # the reference's factory (lib/networks/make_network.py)
 assert type(net).__module__ == ours and os.path.samefile(sys.modules[ours].__file__, ours + ".py"), type(net)
-ref_mod = importlib.import_module({ref_module!r})            # the reference's own class for the same cfg
-torch.manual_seed(0)
-ref = ref_mod.Network()
-a, b = net.state_dict(), ref.state_dict()
-assert list(a.keys()) == list(b.keys()), set(a) ^ set(b)
-for k in a:
-    assert a[k].shape == b[k].shape and a[k].dtype == b[k].dtype, k
-    assert torch.equal(a[k], b[k]), "same seed -> same initial weights: " + k
-net.load_state_dict(b, strict=True)                        # what lib/utils/net_utils.py:load_network does with latest.pth
-ref.load_state_dict(a, strict=True)
+a = net.state_dict()
+got, want = state_dict_digest(a), fx["state_dict"]
+assert [g[0] for g in got] == [w[0] for w in want], set(g[0] for g in got) ^ set(w[0] for w in want)
+for g, w in zip(got, want):
+    assert g[1:3] == w[1:3], (g[:3], w[:3])
+    assert g[3] == w[3], "same seed -> same initial weights: " + g[0]
+ref_sd = {{k: torch.zeros(shape, dtype=getattr(torch, dtype)) for k, shape, dtype, _ in want}}
+net.load_state_dict(ref_sd, strict=True)                   # what lib/utils/net_utils.py:load_network does with latest.pth
+assert all(not v.any() for v in net.state_dict().values())
 import enerf_b200.config as bcfg
 assert bcfg.get_cfg() is cfg                               # the plugin reads the reference's global cfg, not a private copy
 assert next(net.parameters()).device.type == "cpu" and callable(getattr(net, "forward"))
@@ -58,12 +61,9 @@ print("BOUNDARY_OK", len(a))
 '''
 
 
-@pytest.mark.parametrize("variant", sorted(VARIANTS))
+@pytest.mark.parametrize("variant", VARIANTS)
 def test_reference_make_network_loads_the_plugin(variant):
-    if find_reference() is None:
-        pytest.skip("reference tree not available (GPU box): the judge-reproducible check runs in the authoring container")
-    yaml, ref_module, opts = VARIANTS[variant]
-    code = CHILD.format(root=ROOT, variant=variant, yaml=yaml, opts=opts, ref_module=ref_module)
+    code = CHILD.format(root=ROOT, variant=variant)
     env = dict(os.environ)
     env.pop("ENERF_B200_PRECISION", None)
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300, env=env)
